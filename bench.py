@@ -1,6 +1,6 @@
 """Benchmark of the hot path: one G+D training step's worth of torch_utils.ops calls.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload lres|sres] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload lres|sres] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" replays, through this repository's public ops (torch_utils.ops.* -> C ABI -> sm_100a
 kernels), every hot-path operator call that one LongVideoGAN training step issues, at the real
@@ -22,6 +22,13 @@ in HBM; `e2e` = the same with the step's real-video batch copied from pinned hos
 the result read back inside the timed region; `roofline` = achieved algorithmic HBM GB/s of the
 dominant kernel (bias_act), timed with CUDA events inside the timed steps; `cpu_baseline` = the
 CPU oracle (oracle/, a port of the reference's _ref path) on a bounded sample, reported only.
+
+Inputs are seeded: with the same arguments every run replays the same tensors. --dump-outputs DIR writes, after the
+timed steps, what the last timed step of each measured run computed -- a fixed, seeded sample (OutputSampler.N elements)
+of every output and gradient the replayed calls hand back, and of the optimiser's parameters -- as float32
+DIR/<run>.<net>.<call>_<op>.<what>.npy, so that two builds can be compared output for output. The sample is gathered on
+the device inside the step (CUDA graphs included), which adds small gather launches to every step timed in that mode
+-- the e2e and eager figures of a dump run as well as `value`; runs without --dump-outputs have none.
 """
 import argparse
 import json
@@ -29,6 +36,7 @@ import os
 import subprocess
 import sys
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, 'long-video-gan_b200'))
@@ -79,24 +87,51 @@ def scaled(shape, batch):
 # our arm: replay through torch_utils.ops on the GPU
 
 def run_backward(y, leaves, dy):
-    """Backward of ONE replayed call. A training step calls loss.backward() once; replaying the calls one by one
-    would pay torch.autograd.grad's Python-side argument validation (~50 us) per call, which is harness overhead,
-    not operator cost -- so the autograd engine is entered directly (what torch.autograd.grad does after validating)."""
+    """Backward of ONE replayed call -> the gradients of `leaves`. A training step calls loss.backward() once; replaying
+    the calls one by one would pay torch.autograd.grad's Python-side argument validation (~50 us) per call, which is
+    harness overhead, not operator cost -- so the autograd engine is entered directly (what torch.autograd.grad does
+    after validating)."""
     try:
-        torch.autograd.variable.Variable._execution_engine.run_backward(
+        return torch.autograd.variable.Variable._execution_engine.run_backward(
             (y,), (dy,), False, False, tuple(leaves), allow_unreachable=True, accumulate_grad=False)
     except (AttributeError, TypeError):
-        torch.autograd.grad(y, leaves, dy, allow_unused=True)
+        return torch.autograd.grad(y, leaves, dy, allow_unused=True)
+
+
+class OutputSampler:
+    """Gathers a fixed sample of every tensor handed to `keep` into a float32 device buffer per key (one take + one copy
+    launch, so it can sit inside a captured graph). The sample positions of a key are drawn, seeded by the key, when the
+    key is first seen -- in an eager warm-up step, before any capture."""
+    N = 4096
+
+    def __init__(self, prefix):
+        self.prefix = prefix
+        self.idx, self.buf = {}, {}
+
+    def keep(self, key, t):
+        if t is None:
+            return
+        key = self.prefix + key
+        if key not in self.idx:
+            n = t.numel()
+            sel = np.sort(np.random.default_rng(zlib.crc32(key.encode())).choice(n, min(n, self.N), replace=False))
+            self.idx[key] = torch.from_numpy(sel).to(t.device)
+            self.buf[key] = torch.empty(len(sel), dtype=torch.float32, device=t.device)
+        self.buf[key].copy_(torch.take(t.detach(), self.idx[key]))
+
+    def snapshot(self):
+        return {k: v.cpu().numpy() for k, v in self.buf.items()}
 
 
 class Replay:
-    def __init__(self, calls, batch, device, dtype_policy, ops=None):
+    def __init__(self, calls, batch, device, dtype_policy, ops=None, tag=''):
         if ops is None:
             from torch_utils.ops import bias_act, upfirdn2d, filtered_lrelu, conv2d_resample, conv2d_gradfix, conv_nd
             ops = dict(bias_act=bias_act, upfirdn2d=upfirdn2d, filtered_lrelu=filtered_lrelu, conv2d_resample=conv2d_resample,
                        conv2d=conv2d_gradfix, conv3d=conv_nd.conv3d, conv1d=conv_nd.conv1d)
         self.ops = ops
         self.last_y = None
+        self.sampler = None          # an OutputSampler when the outputs are dumped
         self.device = device
         self.pool = {}
         self.items = []
@@ -107,13 +142,13 @@ class Replay:
                 # modulated convolution: the batch lives in the groups (x [1, G*Cin, H, W], w [G*Cout, Cin, k, k])
                 xs = [1, c['x'][1] * batch] + list(c['x'][2:])
                 x = self._buf('x', xs, dt)
-                item = dict(c=c, x=x, dtype=dt, groups=c['groups'] * batch)
+                item = dict(c=c, x=x, dtype=dt, groups=c['groups'] * batch, key=f"{tag}{len(self.items):03d}_{c['op']}")
                 ws = [c['w'][0] * batch] + list(c['w'][1:])
                 item['w'] = (torch.randn(*ws, device=device) / np.sqrt(np.prod(c['w'][1:]))).to(dt)
                 self.items.append(item)
                 continue
             x = self._buf('x', scaled(c['x'], batch), dt)
-            item = dict(c=c, x=x, dtype=dt)
+            item = dict(c=c, x=x, dtype=dt, key=f"{tag}{len(self.items):03d}_{c['op']}")
             if c['op'] in CONV_OPS:
                 item['w'] = (torch.randn(*c['w'], device=device) / np.sqrt(np.prod(c['w'][1:]))).to(dt)
                 item['nograd'] = c['groups'] > 1          # BlurredNoise.blur: fixed filters on a noise input (generator_lres.py:378-387)
@@ -168,29 +203,38 @@ class Replay:
         return self.ops['conv2d_resample'].conv2d_resample(x, it['w'], f=it['f'], up=c['up'], down=c['down'], padding=c['padding'],
                                                            groups=c['groups'], flip_weight=c['flip_weight'], flip_filter=c['flip_filter'])
 
+    def _keep(self, it, what, t):
+        if self.sampler is not None:
+            self.sampler.keep(f"{it['key']}.{what}", t)
+
     def forward_only(self):
         with torch.no_grad():
             for it in self.items:
                 self.last_y = self._fwd(it, it['x'])
+                self._keep(it, 'y_nograd', self.last_y)
 
     def forward_backward(self, timer=None, lo=0, hi=None):
         for it in self.items[lo:hi]:
             if it.get('nograd'):
                 with torch.no_grad():
                     self.last_y = self._fwd(it, it['x'])
+                self._keep(it, 'y', self.last_y)
                 continue
             x = it['x'].detach().requires_grad_(True)
-            leaves = [x]
+            leaves, names = [x], ['dx']
             b = it.get('b')
             if b is not None:
                 b = b.detach().requires_grad_(True)
                 leaves.append(b)
+                names.append('db')
             saved_b = it.get('b')
             it['b'] = b
             saved_w = it.get('w')
             if saved_w is not None:
                 it['w'] = saved_w.detach().requires_grad_(True)
                 leaves.append(it['w'])
+                names.append('dw')
+            grads = ()
             if timer is not None and it['c']['op'] in timer.ops:
                 flops = it.get('flops_fwd')
                 timer.start()
@@ -198,13 +242,16 @@ class Replay:
                 timer.stop(it['bytes_fwd_grad'] if flops is None else flops)
                 if y.requires_grad:
                     timer.start()
-                    run_backward(y, leaves, it['dy'])
+                    grads = run_backward(y, leaves, it['dy'])
                     timer.stop(it['bytes_bwd'] if flops is None else 2.0 * flops)
             else:
                 y = self._fwd(it, x)
                 if y.requires_grad:
-                    run_backward(y, leaves, it['dy'])
+                    grads = run_backward(y, leaves, it['dy'])
             self.last_y = y.detach()
+            self._keep(it, 'y', self.last_y)
+            for name, g in zip(names, grads):
+                self._keep(it, name, g)
             it['b'] = saved_b
             if saved_w is not None:
                 it['w'] = saved_w
@@ -584,16 +631,20 @@ class GradExchange:
 
 # ---------------------------------------------------------------------------------------------
 
-def run_ours(args, workload, scope, steps, rank, world, local_rank, device, with_cpu, with_refcuda):
-    """One workload through this repository's ops on the GPU -> the JSON fields of its line."""
+def run_ours(args, workload, scope, steps, rank, world, local_rank, device, with_cpu, with_refcuda, dump=None):
+    """One workload through this repository's ops on the GPU -> the JSON fields of its line. `dump` (a dict): receives
+    the sampled outputs of the last step of the main timed region, keyed '<workload>.<scope>.<net><call>_<op>.<what>'."""
     global _scope
     import torch.distributed as dist
     from torch_utils import custom_ops
     _scope = scope
+    torch.manual_seed(0)                     # the same inputs in every run with the same arguments
     g_calls, d_calls, batch, frames = load_trace(workload)
     policy = 'mixed' if workload == 'sres' else 'fp32'
-    G = Replay(g_calls, batch, device, policy)
-    D = Replay(d_calls, batch, device, policy)
+    G = Replay(g_calls, batch, device, policy, tag='G')
+    D = Replay(d_calls, batch, device, policy, tag='D')
+    outputs = OutputSampler(f'{workload}.{scope}.') if dump is not None else None
+    G.sampler = D.sampler = outputs
     kBuckets = 4
     ex_g = ex_d = None
     if world > 1:
@@ -726,6 +777,14 @@ def run_ours(args, workload, scope, steps, rank, world, local_rank, device, with
     sampler = ClockSampler(local_rank) if rank == 0 else None
     timer = KernelTimer(dominant_op)
     ms_total = timed(steps, e2e=False, timer=None if graphs else timer)
+    if outputs is not None:
+        # the optimiser's state after the last timed step (sampled outside the timed region), then everything kept so far
+        tails = (tail_g, tail_d) if world == 1 else (ex_g.tail, ex_d.tail)
+        for net, tail in zip('GD', tails):
+            outputs.keep(f'{net}.adam.params', tail.opt.flat_params)
+            outputs.keep(f'{net}.adam.ema', tail.ema_flat)
+        dump.update(outputs.snapshot())
+        G.sampler = D.sampler = None
     launches = launches_per_step * steps if graphs else custom_ops.launch_count() - launches0
     step(e2e=True)                           # untimed warm-up of the host-copy flavour
     ms_e2e = timed(steps, e2e=True)
@@ -844,7 +903,9 @@ def run_ours(args, workload, scope, steps, rank, world, local_rank, device, with
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=10,
+                    help="timed steps of each of this repository's runs (lres, ops_only, sres); the ref_cuda comparison times 2..5 steps "
+                         "and --impl reference samples up to K steps within a ~3-minute guard")
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--workload', default='both', choices=sorted(WORKLOADS) + ['both'],
                     help="both (default): the line's value is the lres step (BASELINE configs[1]); the sres step (configs[2]) is measured in the same run and reported under the key sres")
@@ -859,7 +920,13 @@ def main():
     ap.add_argument('--no-ref-cuda', action='store_true')
     ap.add_argument('--launch', default='graph', choices=['graph', 'eager'],
                     help='graph: the step is captured once into CUDA graphs and replayed (default); eager: every call launched from Python')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write a fixed sample of what the last timed step computed (outputs, gradients, optimiser state) as DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
 
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -909,15 +976,24 @@ def main():
     from torch_utils import custom_ops
     custom_ops.load_library()
 
-    res = run_ours(args, primary, args.scope, args.steps, rank, world, local_rank, device, with_cpu=not args.no_cpu, with_refcuda=not args.no_ref_cuda)
+    dump = {} if args.dump_outputs else None
+    res = run_ours(args, primary, args.scope, args.steps, rank, world, local_rank, device, with_cpu=not args.no_cpu, with_refcuda=not args.no_ref_cuda,
+                   dump=dump)
     sres = ops_only = None
     if args.workload == 'both':
         torch.cuda.empty_cache()
         if args.scope == 'full':
-            ops_only = run_ours(args, primary, 'ops', args.steps, rank, world, local_rank, device, with_cpu=False, with_refcuda=not args.no_ref_cuda)
+            ops_only = run_ours(args, primary, 'ops', args.steps, rank, world, local_rank, device, with_cpu=False, with_refcuda=not args.no_ref_cuda,
+                                dump=dump)
             torch.cuda.empty_cache()
-        sres = run_ours(args, 'sres', 'ops', max(2, min(args.steps, 5)), rank, world, local_rank, device, with_cpu=False,
-                        with_refcuda=not args.no_ref_cuda)
+        sres = run_ours(args, 'sres', 'ops', args.steps, rank, world, local_rank, device, with_cpu=False, with_refcuda=not args.no_ref_cuda,
+                        dump=dump)
+    if dump is not None and rank == 0:
+        nbytes = sum(a.nbytes for a in dump.values())
+        assert nbytes <= 64 << 20, f'--dump-outputs: {nbytes} bytes of samples, more than 64 MB'
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, k + '.npy'), a)
     if rank == 0:
         out = {'metric': metric, 'value': res['value'], 'unit': 'frames/s', 'n_gpus': world, 'steps': args.steps, 'warmup': res['warmup'],
                'ms_per_step': res['ms_per_step'], 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
